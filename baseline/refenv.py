@@ -1,8 +1,8 @@
 """Locates and imports the UNMODIFIED reference for tests and bench.py's reference arms.
 
-The reference lives under baseline/_ref/ (installed by baseline/install_ref.py; git-ignored, ships
-to the GPU box with gpurun).  Test / benchmark infrastructure only: nothing under fuxictr_b200/
-imports this module, and nothing here reads /root/reference.
+The reference lives under oracle/_ref/ (installed from a FuxiCTR checkout by oracle/install_ref.py,
+which __graft_entry__.build() runs; git-ignored).  Test / benchmark infrastructure only: nothing under
+fuxictr_b200/ imports this module, and nothing here reads the checkout itself.
 
 SURVEY.md 8(c): `import fuxictr.pytorch.layers` needs three import-time-only dependencies that the
 offline image lacks (h5py, polars, keras_preprocessing); empty stub modules are inserted for the
@@ -16,7 +16,7 @@ import sys
 import types
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF_ROOT = os.path.join(HERE, "_ref")
+REF_ROOT = os.path.join(os.path.dirname(HERE), "oracle", "_ref")
 EXTRAS = os.path.join(REF_ROOT, "extras")
 
 MODEL_DIRS = {
@@ -33,7 +33,7 @@ def available():
 
 
 def why_unavailable():
-    return "baseline/_ref is missing (run `python baseline/install_ref.py` in the build container)"
+    return "oracle/_ref is missing (build() installs it when a FuxiCTR checkout is found; see oracle/install_ref.py)"
 
 
 _IMPORTED = {}
@@ -58,7 +58,7 @@ def import_reference():
         sys.path.insert(0, REF_ROOT)
     import fuxictr
     if not os.path.abspath(fuxictr.__file__).startswith(REF_ROOT):
-        raise ImportError("another `fuxictr` (%s) shadows baseline/_ref" % fuxictr.__file__)
+        raise ImportError("another `fuxictr` (%s) shadows oracle/_ref" % fuxictr.__file__)
     import fuxictr.pytorch.layers as layers
     from fuxictr.features import FeatureMap
     from fuxictr.pytorch.models.rank_model import BaseModel

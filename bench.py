@@ -13,7 +13,7 @@ interaction / MLP forward -> BCE -> backward (dense-gradient scatter-add, GEMM d
 clip_grad_norm_(10) -> Adam over every parameter.
 
     python bench.py --gpus N --steps K --warmup W          # this repo's CUDA path
-    python bench.py --impl reference ...                   # the UNMODIFIED reference (baseline/_ref) on host CPU
+    python bench.py --impl reference ...                   # the UNMODIFIED reference (oracle/_ref) on host CPU
     python bench.py --impl reference-gpu ...               # the unmodified reference, eager, on cuda:0
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for every field.
@@ -65,7 +65,19 @@ def parse():
     ap.add_argument("--precision", default="tf32x3", choices=["fp32", "tf32x3", "tf32", "bf16"],
                     help="arithmetic of the dense GEMMs: fp32 FFMA, 3xTF32 (fp32-class, the parity mode), 1xTF32, or "
                          "bf16 operands with fp32 accumulation (BASELINE configs[1]) on tcgen05")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned and left behind (its loss and "
+                         "the model's floating-point state_dict; --gpus 1) as DIR/<name>.npy; large tensors keep a "
+                         "fixed, seeded sample of distinct rows, first those the last timed batch touched, so that the "
+                         "dump stays under 64 MB.  The inputs are the same "
+                         "on every run, but the backward accumulates with float atomics: two runs agree to rounding "
+                         "after the first steps and drift apart as steps add up, so compare builds at a small --steps")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "b200":
+        raise SystemExit("--dump-outputs dumps the b200 arm's training step (--impl b200)")
+    if a.dump_outputs and a.gpus != 1:
+        raise SystemExit("--dump-outputs dumps one GPU's training step (--gpus 1): a row-sharded rank holds a "
+                         "slice of the tables and of the batch")
     if a.batch <= 0:
         a.batch = DEFAULT_BATCH[a.workload] if a.workload != "dlrm" else max(DLRM_GLOBAL_BATCH // max(a.gpus, 1), 1)
     if a.gpus > 1 and a.workload not in ("deepfm", "dlrm"):
@@ -234,9 +246,9 @@ class ClockSampler(object):
 
 
 # ------------------------------------------------------------------------------------------
-# Reference arms: the UNMODIFIED reference from baseline/_ref (its own model class, its own
+# Reference arms: the UNMODIFIED reference from oracle/_ref (its own model class, its own
 # BaseModel.train_step), on the host CPU or eager on cuda:0.  Falls back to the oracle port when
-# baseline/_ref is absent.
+# oracle/_ref is absent.
 # ------------------------------------------------------------------------------------------
 def build_reference_model(args, gpu):
     """(model, feature_map) of the reference's own class for the workload, from a synthetic FeatureMap."""
@@ -290,7 +302,7 @@ def cpu_reference_run(args, steps, warmup, seconds=None, threads=None):
         step = model.train_step
         batches = reference_batches(fm, make_batches(4, batch, specs=make_specs(args)))
         kind = "reference"
-    except ImportError:       # no baseline/_ref on this machine: the oracle restatement (same ATen ops)
+    except ImportError:       # no oracle/_ref on this machine: the oracle restatement (same ATen ops)
         import torch
         from oracle import fuxictr_oracle as O
         from fuxictr_b200 import zoo
@@ -348,7 +360,7 @@ def cpu_reference_run(args, steps, warmup, seconds=None, threads=None):
 
 
 def cpu_baseline_entry(r, args, how):
-    what = ("the unmodified reference (baseline/_ref: model_zoo class + BaseModel.train_step)" if r["kind"] == "reference"
+    what = ("the unmodified reference (oracle/_ref: model_zoo class + BaseModel.train_step)" if r["kind"] == "reference"
             else "oracle port of the reference's ATen path")
     return {"value": r["value"], "unit": "samples/s", "cores": r["cores"], "kind": r["kind"],
             "sample": "%d train steps of batch %d %s on %d of %d host threads (fastest of the sweep %s); %s"
@@ -359,7 +371,7 @@ def run_reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps = min(args.steps, 200)       # bounded: each step is one batch; the run ends within a few minutes
+    steps = args.steps
     warm = min(args.warmup, 5)
     r = cpu_reference_run(args, steps, warm)
     line = {"impl": "reference", "metric": METRICS[args.workload], "value": r["value"], "unit": "samples/s",
@@ -404,7 +416,7 @@ def reference_gpu_eager(args, steps=30, warmup=5):
 def run_reference_gpu_arm(args):
     if int(os.environ.get("RANK", "0")) != 0:
         return
-    r = reference_gpu_eager(args, steps=min(args.steps, 100), warmup=max(min(args.warmup, 10), 3))
+    r = reference_gpu_eager(args, steps=args.steps, warmup=max(min(args.warmup, 10), 3))
     print(json.dumps({"impl": "reference-gpu", "metric": METRICS[args.workload], "value": r["value"],
                       "unit": "samples/s", "n_gpus": 1, "higher_is_better": True, "dtype": "f32", "data": "synthetic",
                       "config": workload_config(args, 1), "detail": r}))
@@ -588,6 +600,60 @@ def gather_points(peaks, rows, vs_label):
             "points": res}
 
 
+DUMP_BYTES = 60 << 20          # under the 64 MB that --dump-outputs promises
+
+
+def touched_rows(fm, batch, key):
+    """Rows of the embedding table `key` (a state_dict key) that the batch matrix indexes, or None."""
+    import torch
+    if not key.endswith(".weight") or "embedding_layers." not in key:
+        return None
+    table = key.split("embedding_layers.")[-1][:-len(".weight")]
+    cols = []
+    for name, sp in fm.features.items():
+        if name == table or sp.get("share_embedding") == table:
+            idx = fm.column_index[name]
+            cols += idx if isinstance(idx, list) else [idx]
+    return batch[:, cols].long().flatten().unique() if cols else None
+
+
+def sample_rows(nrows, n, gen, touched=None):
+    """n distinct row indices out of nrows (n < nrows): rows in `touched` first, the rest uniform."""
+    import torch
+    pick = torch.empty(0, dtype=torch.long)
+    if touched is not None:
+        pick = touched[torch.randperm(len(touched), generator=gen)[:n]]
+    if len(pick) < n:
+        rest = (torch.randperm(nrows, generator=gen) if nrows <= 4 * n
+                else torch.randint(0, nrows, (2 * n,), generator=gen).unique())
+        rest = rest[~torch.isin(rest, pick)]
+        pick = torch.cat([pick, rest[torch.randperm(len(rest), generator=gen)[:n - len(pick)]]])
+    return pick.sort().values
+
+
+def dump_outputs(out_dir, loss, model, fm, last_batch):
+    """Writes the last timed step's loss and the floating-point state_dict it left as
+    out_dir/<name>.npy (float32, float64 kept as such).  An array larger than its even share of
+    DUMP_BYTES keeps a sample of distinct rows drawn from a generator seeded with its position in the
+    state_dict, embedding tables first from the rows `last_batch` (the last timed step's input)
+    updated: the same rows every run, so that two builds can be compared array for array."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    params = [(k, v.detach()) for k, v in model.state_dict().items() if v.is_floating_point()]
+    share = DUMP_BYTES // (len(params) + 1)
+    arrays = [("loss", torch.tensor([loss], dtype=torch.float32))]
+    for i, (k, v) in enumerate(params):
+        cap = share // (8 if v.dtype == torch.float64 else 4)
+        if v.numel() > cap:
+            n = max(cap // max(v[0].numel(), 1), 1)
+            rows = sample_rows(v.shape[0], n, torch.Generator().manual_seed(i), touched_rows(fm, last_batch, k))
+            v = v.index_select(0, rows.to(v.device))
+        arrays.append(("param." + k, v.double() if v.dtype == torch.float64 else v.float()))
+    for name, v in arrays:
+        np.save(os.path.join(out_dir, name + ".npy"), v.cpu().numpy())
+
+
 def load_peaks():
     path = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(path):
@@ -744,6 +810,8 @@ def run_b200_arm(args):
     ms_total = timed(False, args.steps, warmup)
     ms_e2e = timed(True, args.steps, warmup)
     t_w1 = time.time()
+    if args.dump_outputs and rank == 0:     # before the untimed clock-sampling steps below change the state
+        dump_outputs(args.dump_outputs, pipe.loss(), model, fm, host_batches[(warmup + args.steps - 1) % len(host_batches)])
     windows, clock_note = [(t_w0, t_w1)], "rows sampled inside the two timed regions"
     if ms_total + ms_e2e < 600.0:
         # a few hundred sub-millisecond steps end before nvidia-smi's 100 ms sampling sees them: keep the
@@ -847,7 +915,7 @@ def run_b200_arm(args):
         except Exception as exc:  # e.g. a smaller GPU: report, do not hide
             line["gather"] = {"error": str(exc)}
         try:
-            line["reference_gpu_eager"] = reference_gpu_eager(args)
+            line["reference_gpu_eager"] = reference_gpu_eager(args, steps=args.steps)
         except Exception as exc:
             line["reference_gpu_eager"] = {"unavailable": repr(exc)}
     if world == 1 and not args.no_cpu_baseline and args.workload != "dlrm":

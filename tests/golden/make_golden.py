@@ -378,6 +378,27 @@ def case_init_parity():
                                   "kwargs": dict(embedding_dim=4, hidden_units=[8, 8])}, w=sd(model))
 
 
+def case_mirror_constructors():
+    """state_dict and module tree of the model_zoo classes right after construction with seed 4242,
+    for every configuration of tests/test_host_logic.py:_MIRROR_CASES (one group per case)."""
+    tests_dir = os.path.dirname(HERE)
+    sys.path[:0] = [tests_dir, os.path.dirname(tests_dir)]
+    from test_host_logic import _MIRROR_CASES, _mirror_case_ids
+    rel = {"DeepFM": "DeepFM/DeepFM_torch", "DCNv2": "DCNv2", "DLRM": "DLRM", "DIN": "DIN", "xDeepFM": "xDeepFM"}
+    meta, groups = {"seed": 4242, "cases": {}}, {}
+    for case_id, (name, specs, kwargs) in zip(_mirror_case_ids(), _MIRROR_CASES):
+        cls = load_model_class(rel[name], name)
+        torch.manual_seed(4242)
+        model = cls(synthetic_fm(specs, emb_dim=kwargs["embedding_dim"]), model_root="/tmp/b2_mirror/", metrics=["AUC"],
+                    verbose=0, gpu=-1, optimizer="adam", loss="binary_crossentropy", **kwargs)
+        w = sd(model)
+        modules = [[m, "%s.%s" % (type(mod).__module__, type(mod).__qualname__)
+                    if type(mod).__module__.startswith("torch.") else None] for m, mod in model.named_modules()]
+        meta["cases"][case_id] = {"keys": list(w.keys()), "modules": modules}
+        groups[case_id] = w
+    save("mirror_constructors_seed4242", meta, **groups)
+
+
 def case_next_layers():
     """Layers of the "next" row 8f-4 (kernels not built yet): pins the oracle restatement first."""
     import fuxictr.pytorch.layers as LL
@@ -470,6 +491,9 @@ if __name__ == "__main__":
     if "--only-next" in sys.argv:
         case_next_layers()
         sys.exit(0)
+    if "--only-mirror" in sys.argv:
+        case_mirror_constructors()
+        sys.exit(0)
     case_feature_embedding_tiny_npz()
     case_feature_embedding_dict_tiny_seq()
     case_logistic_regression_tiny_seq()
@@ -479,5 +503,6 @@ if __name__ == "__main__":
     case_mlp_dice_din()
     case_models()
     case_init_parity()
+    case_mirror_constructors()
     case_metrics()
     case_next_layers()

@@ -7,7 +7,8 @@
    (npz: one named array per column, sequences as (N, L) arrays; parquet: list-valued cells);
 2. runs the REAL reference loaders (fuxictr.pytorch.dataloaders, imported from /root/reference —
    build container only) over them with a fixed torch seed and stores per-case SHA-256 digests of
-   every batch in tests/golden/loader_digests.json (cases: tests/test_dataloader.py:CASES).
+   the batches (all of them, each one, and two further shuffled epochs), their keys, dtypes and shapes in
+   tests/golden/loader_digests.json (cases: tests/test_dataloader.py:CASES).
 """
 import hashlib
 import json
@@ -99,9 +100,15 @@ def reference_digests():
         torch.manual_seed(7)
         loader = cls(fm, os.path.join(DATA, dataset, split), batch_size=batch_size, shuffle=shuffle, num_workers=0)
         batches = list(loader)
-        out["%s/%s/%s/%d/%d" % (dataset, fmt, split, batch_size, int(shuffle))] = {
-            "sha256": digest(batches), "num_batches": len(loader), "num_samples": loader.num_samples,
-            "dtype": str(batches[0][fm.labels[0]].dtype)}
+        entry = {"sha256": digest(batches), "num_batches": len(loader), "num_samples": loader.num_samples,
+                 "dtype": str(batches[0][fm.labels[0]].dtype),
+                 "keys": list(batches[0].keys()), "dtypes": {k: str(v.dtype) for k, v in batches[0].items()},
+                 "batch_shapes": [[list(v.shape) for v in b.values()] for b in batches],
+                 "batch_sha256": [digest([b]) for b in batches]}
+        if shuffle:     # the next two epochs after reseeding: the permutation stream of the loader
+            torch.manual_seed(11)
+            entry["two_epochs_seed11_sha256"] = digest([b for _ in range(2) for b in loader])
+        out["%s/%s/%s/%d/%d" % (dataset, fmt, split, batch_size, int(shuffle))] = entry
     with open(os.path.join(HERE, "loader_digests.json"), "w") as fd:
         json.dump(out, fd, indent=1, sort_keys=True)
     print("wrote", len(out), "digests")

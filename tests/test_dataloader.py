@@ -1,5 +1,5 @@
-"""fuxictr_b200.dataloader on the CPU: batches equal the REAL reference loaders' batches (build
-container only), the golden digests of those batches (everywhere), and the structural contract
+"""fuxictr_b200.dataloader on the CPU: batches equal the REAL reference loaders' batches (where the
+reference is installed), the stored digests of those batches (everywhere), and the structural contract
 (num_samples / num_batches / len / RankDataLoader stages).  Pure host logic: no GPU."""
 import hashlib
 import json
@@ -13,7 +13,7 @@ import torch
 
 from conftest import GOLDEN, ROOT
 
-from baseline import refenv  # noqa: E402  (the unmodified reference under baseline/_ref)
+from baseline import refenv  # noqa: E402  (the unmodified reference under oracle/_ref)
 HAVE_REF = refenv.available()
 FIXTURES = os.path.join(ROOT, "tests", "golden", "data")
 
@@ -95,6 +95,27 @@ def test_batches_match_the_live_reference(ref_loaders, dataset, fmt, split, batc
         torch.manual_seed(11)
         got2 = [b for _ in range(2) for b in loader]
         assert _digest(got2) == _digest(want2)
+
+
+@pytest.mark.parametrize("dataset,fmt,split,batch_size,shuffle", CASES)
+def test_batches_match_the_stored_reference_batches(dataset, fmt, split, batch_size, shuffle):
+    """The live comparison above, against what the reference's own loaders yielded when the goldens
+    were made (keys, dtypes, shapes and SHA-256 of every batch; make_loader_golden.py): runs without
+    the reference installed."""
+    with open(os.path.join(GOLDEN, "loader_digests.json")) as fd:
+        want = json.load(fd)["%s/%s/%s/%d/%d" % (dataset, fmt, split, batch_size, int(shuffle))]
+    loader, got = _ours(dataset, fmt, split, batch_size, shuffle)
+    assert len(got) == len(want["batch_sha256"]) == len(loader) == want["num_batches"]
+    for a, shapes, digest in zip(got, want["batch_shapes"], want["batch_sha256"]):
+        assert list(a.keys()) == want["keys"]
+        assert {k: str(v.dtype) for k, v in a.items()} == want["dtypes"]
+        assert [list(v.shape) for v in a.values()] == shapes
+        assert _digest([a]) == digest
+    # a second epoch draws the next permutation from the same RNG stream on both sides
+    if shuffle:
+        torch.manual_seed(11)
+        got2 = [b for _ in range(2) for b in loader]
+        assert _digest(got2) == want["two_epochs_seed11_sha256"]
 
 
 def test_matrices_are_the_collators_matrix():

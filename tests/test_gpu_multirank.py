@@ -1,7 +1,6 @@
 """Row-sharded training over REAL ranks (one process per GPU, NVLink peer memory + NCCL): launched with
-torchrun when the box has >= 2 GPUs (the driver's single-GPU `-m gpu` run skips it; the builder runs
-it under `gpurun --gpus 2/8`, logs in profiles/).  The script compares against the CPU oracle on the
-global batch (tools/dist_sharded_check.py)."""
+torchrun when the machine has >= 2 GPUs (skipped on a single GPU; logs of 2- and 8-GPU runs in
+profiles/).  The script compares against the CPU oracle on the global batch (tools/dist_sharded_check.py)."""
 import os
 import subprocess
 import sys
@@ -23,7 +22,7 @@ def _ngpus():
 def test_sharded_training_matches_the_oracle_on_real_ranks(model, precision):
     n = _ngpus()
     if n < 2:
-        pytest.skip("needs >= 2 GPUs (run under `gpurun --gpus 2`)")
+        pytest.skip("needs >= 2 GPUs")
     world = 8 if n >= 8 else (4 if n >= 4 else 2)
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", str(world),
            "--master-addr", "127.0.0.1", "--master-port", "29611", os.path.join(ROOT, "tools", "dist_sharded_check.py"),

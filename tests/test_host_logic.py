@@ -130,8 +130,10 @@ def test_batch_views_alias_the_matrix_for_sequences_too():
 
 
 # ---------------------------------------------------------------------------------------------
-# Mirror constructors vs the LIVE reference (baseline/_ref): same seed => bit-identical state_dict
+# Mirror constructors vs the LIVE reference (oracle/_ref): same seed => bit-identical state_dict
 # (keys, shapes, registration order, RNG consumption order), over more configurations than the goldens.
+# The same comparison against the stored reference state (mirror_constructors_seed4242.npz, made by
+# tests/golden/make_golden.py) runs without the reference installed.
 # ---------------------------------------------------------------------------------------------
 _SEQ_SPECS = [
     ("user", {"type": "categorical", "source": "", "padding_idx": 0, "vocab_size": 30}),
@@ -168,7 +170,11 @@ _MIRROR_CASES = [
 ]
 
 
-@pytest.mark.parametrize("name,specs,kwargs", _MIRROR_CASES, ids=["%s-%d" % (c[0], i) for i, c in enumerate(_MIRROR_CASES)])
+def _mirror_case_ids():
+    return ["%s-%d" % (c[0], i) for i, c in enumerate(_MIRROR_CASES)]
+
+
+@pytest.mark.parametrize("name,specs,kwargs", _MIRROR_CASES, ids=_mirror_case_ids())
 def test_mirror_constructors_match_the_live_reference_seed_for_seed(name, specs, kwargs):
     from baseline import refenv
     if not refenv.available():
@@ -192,4 +198,26 @@ def test_mirror_constructors_match_the_live_reference_seed_for_seed(name, specs,
         assert mname in ref_mods, mname
         if type(ref_mods[mname]).__module__.startswith("torch."):
             assert type(mod) is type(ref_mods[mname]), mname
+    assert set(ref_mods) == set(dict(ours.named_modules()))
+
+
+@pytest.mark.parametrize("name,specs,kwargs", _MIRROR_CASES, ids=_mirror_case_ids())
+def test_mirror_constructors_match_the_stored_reference_seed_for_seed(request, name, specs, kwargs):
+    g = Golden("mirror_constructors_seed4242")
+    case = g.meta["cases"][request.node.callspec.id]
+    sd_ref = g[request.node.callspec.id]
+    torch.manual_seed(g.meta["seed"])
+    ours = getattr(zoo, name)(FeatureMap.from_specs(specs, embedding_dim=kwargs["embedding_dim"]), gpu=-1, **kwargs)
+    sd = ours.state_dict()
+    assert list(sd.keys()) == case["keys"]
+    for k in case["keys"]:
+        v = sd_ref[k]
+        assert sd[k].dtype == v.dtype and sd[k].shape == v.shape, k
+        assert torch.equal(sd[k], v), k
+    # module tree: same names, and the same torch module type wherever the reference uses a stock one
+    ref_mods = dict(case["modules"])
+    for mname, mod in ours.named_modules():
+        assert mname in ref_mods, mname
+        if ref_mods[mname] is not None:
+            assert "%s.%s" % (type(mod).__module__, type(mod).__qualname__) == ref_mods[mname], mname
     assert set(ref_mods) == set(dict(ours.named_modules()))

@@ -1,4 +1,4 @@
-"""fuxictr_b200.patch.enable() on the REAL reference (baseline/_ref) without a GPU: class identity,
+"""fuxictr_b200.patch.enable() on the REAL reference (oracle/_ref) without a GPU: class identity,
 state_dict and CPU behaviour are untouched, and CUDA tensors would be routed to the kernels.  The
 same boundary on a real device: tests/test_reference_boundary.py (-m gpu)."""
 import os

@@ -1,5 +1,5 @@
 """The REAL drop-in boundary (SURVEY.md 8b / row a15): the unmodified reference installed under
-baseline/_ref (fuxictr package + the five in-scope model_zoo directories + demo/ + data/tiny_*),
+oracle/_ref (fuxictr package + the five in-scope model_zoo directories + demo/ + data/tiny_*),
 its models built from their own `*_test` YAML experiments, its own loaders, its own
 `BaseModel.train_step` / `fit` / `evaluate` — with `fuxictr_b200.patch.enable()` routing the
 layer forwards to the sm_100a kernels when the model sits on cuda:0.
@@ -9,8 +9,8 @@ tensors on the reference's own code).  Bars: forward y_pred and the weights afte
 `train_step`s within 1e-5 relative fp32 (north_star); `call_counts()` proves the kernels ran.
 C1 = demo/example3 end to end (BASELINE configs[0]).
 
-The `gpu` tests need baseline/_ref on the box (it ships with gpurun); the CPU tests check the
-reference environment itself.
+The `gpu` tests need oracle/_ref on the GPU machine (build() installs it from a FuxiCTR checkout and
+it travels with the built tree); the CPU tests check the reference environment itself.
 """
 import logging
 import os
@@ -68,7 +68,7 @@ def first_batches(R, fm, params, n):
 
 
 def test_reference_environment_runs_a_yaml_experiment_on_cpu():
-    """baseline/_ref really is the reference and its YAML entry path works here (CPU)."""
+    """oracle/_ref really is the reference and its YAML entry path works here (CPU)."""
     with tempfile.TemporaryDirectory() as tmp:
         R, params, fm, model = build("DeepFM", "DeepFM_test", "tiny_parquet", -1, tmp)
         assert os.path.abspath(sys.modules["fuxictr"].__file__).startswith(refenv.REF_ROOT)
